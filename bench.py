@@ -3,6 +3,7 @@
 
     python bench.py --gpus 1 --steps 20 --warmup 3                 # B200 arm
     python bench.py --impl reference --steps 20 --warmup 3          # CPU arm (oracle port)
+    python bench.py --gpus 1 --steps 20 --warmup 3 --dump-outputs DIR   # + what the last timed step computed
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W       # weak scaling
 
@@ -280,6 +281,41 @@ def run_c5(sb, rank, world, local, dist, pairs_per_gpu, n_pts):
             "api": "simpleicp_b200.simpleicp_batch(pairs, engine='batched') on pinned host arrays, records all-gathered"}
 
 
+# per-correspondence entries written by --dump-outputs (28 bytes each with the sample index): a
+# larger K is sampled with a fixed seed so that a dump stays under 64 MB
+DUMP_MAX_ENTRIES = 1 << 21
+
+
+def dump_outputs(out_dir: str, eng) -> None:
+    """What the last timed step (one ICP iteration) computed, as the arrays a caller of the
+    iteration receives: the cumulative transform H and parameters x after it, its residual
+    statistics and, per selected fixed point, the matched movable index, the point-to-plane
+    distance and the keep flag of the rejection.  Inputs are seeded, so two builds run with the
+    same arguments can be compared file by file."""
+    rec, H, nn_idx, dist, keep = eng.last_iteration()
+    K = nn_idx.size
+    sample = np.arange(K)
+    if K > DUMP_MAX_ENTRIES:
+        sample = np.sort(np.random.default_rng(0).choice(K, DUMP_MAX_ENTRIES, replace=False))
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    arrays = {
+        "H": H,
+        "x": np.array(rec.x, dtype=np.float64),
+        "n_kept": np.array([rec.n_kept], dtype=np.float64),
+        # median and MAD of the distances, their mean and std, mean and std of the residuals after
+        # the solve, distance weight of the least-squares problem
+        "stats": np.array([rec.median, rec.mad, rec.mean_dist, rec.std_dist, rec.mean_res, rec.std_res,
+                           rec.distance_weight], dtype=np.float64),
+        "sample_index": sample.astype(np.float64),
+        "match_index": nn_idx[sample].astype(np.float64),
+        "distance": dist[sample],
+        "kept": keep[sample].astype(np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
+
+
 def _trace(msg):
     if os.environ.get("SICP_BENCH_TRACE"):
         print(f"[bench rank {os.environ.get('RANK', '0')} t={time.time() % 1000:.1f}] {msg}", file=sys.stderr, flush=True)
@@ -345,6 +381,8 @@ def run_b200(args):
     # the K timed steps: one CUDA-event pair around each whole iteration (cold L2 before each)
     st_outer = eng.time_stages(params, args.steps, True, outer_only=True)
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng)
     launches = eng.timings()["kernel_launches"] - launches0
     # the per-kernel split of the same step, from a second set of steps with events between the
     # kernels (those events cost a few microseconds of stream bubbles, hence not in `value`)
@@ -607,7 +645,11 @@ def main():
     ap.add_argument("--no-c4c5", action="store_true")
     ap.add_argument("--c5-pairs-per-gpu", type=int, default=64)
     ap.add_argument("--c5-points", type=int, default=100_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0 only)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3 if args.impl == "b200" else 0)
     if args.impl == "reference":
         run_reference(args)

@@ -300,6 +300,13 @@ int32_t sicp_get_timings(sicp_ctx* ctx, sicp_timings* t /*[h]*/);
  * bubbles per iteration, so the whole-iteration time is taken without them.                     */
 int32_t sicp_time_stages(sicp_ctx* ctx, const sicp_run_params* p, int32_t reps, int32_t flush_l2,
                          double ms[4] /*[h]*/);
+/* What the last iteration of sicp_iterate or sicp_time_stages computed, read back without
+ * launching anything: its record, the cumulative transform after it, and per selected point the
+ * matched movable index, the point-to-plane distance and the keep flag of the rejection (K entries
+ * each).  Any output may be NULL.  SICP_ERR_STATE once another call has changed the loop state.  */
+int32_t sicp_get_iteration(sicp_ctx* ctx, sicp_iter_record* rec /*[h]*/, double T[16] /*[h]*/,
+                           int64_t* nn_idx /*[h|d] K*/, double* dist /*[h|d] K*/,
+                           uint8_t* keep /*[h|d] K*/);
 /* Diagnostics: %globaltimer stamps block 0 took in the last reject+solve kernel, microseconds
  * relative to kernel entry.  [1] median done, [2] MAD done, [3] moments accumulated, [4] grid
  * barrier passed, [5] LM solve done, [6] barrier, [7] residual pass, [8] barrier, [9] exit;

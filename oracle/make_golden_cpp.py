@@ -1,10 +1,11 @@
 """Generate tests/golden/cppref_<name>.npz by running the UNMODIFIED C++ reference.
 
-Run in the build container only (needs /root/reference and g++):
+Needs g++ and a checkout of pglira/simpleICP (DEFAULT_REFERENCE, or the one $SIMPLEICP_REFERENCE
+names):
 
     python oracle/make_golden_cpp.py            # dragon, bunny, airborne, terrestrial (+ extras)
 
-The C++ tree (/root/reference/c++/src) is the definition of the LINEARISED simpleICP variant
+The C++ tree (c++/src of that checkout) is the definition of the LINEARISED simpleICP variant
 (SURVEY.md section 8f rank 3).  Its sources are compiled where they lie -- never copied -- by
 oracle/Makefile into oracle/_ref/ against stand-in headers for the three third-party libraries
 the image lacks (oracle/cpp_standin: the used subset of Eigen's, nanoflann's and cxxopts'
@@ -14,7 +15,7 @@ pin), exactly as oracle/lmfit_standin does for the Python package.
 Two programs are run per configuration:
 
   * oracle/_ref/simpleicp_cpp -- the reference's own CLI main() -- with the command lines of
-    c++/run_simpleicp.sh on the .xyz files under /root/reference/data: its screen output
+    c++/run_simpleicp.sh on the .xyz files under data/ of the checkout: its screen output
     (iteration table to 4 decimals, H to 6) is stored verbatim (minus the wall-clock line);
   * oracle/_ref/simpleicp_cpp_driver (oracle/cpp_driver.cpp) -- calls the reference's
     SimpleICP() for H with 17 digits and then replays the same sequence of calls on the
@@ -22,10 +23,11 @@ Two programs are run per configuration:
     fails unless both passes end in the bit-identical H.
 
 tests/test_cpp_reference_pin.py checks oracle/linearized_oracle.py against these files (and
-re-runs this recipe when /root/reference is present); tests/test_gpu_linearized.py checks the
+re-runs this recipe where the checkout is readable); tests/test_gpu_linearized.py checks the
 CUDA path against the same files.
 """
 import json
+import os
 import subprocess
 import sys
 import tempfile
@@ -34,7 +36,21 @@ from pathlib import Path
 import numpy as np
 
 REPO = Path(__file__).resolve().parents[1]
-REF = Path("/root/reference")
+# where the fixtures were generated from; $SIMPLEICP_REFERENCE names another checkout
+DEFAULT_REFERENCE = "/root/reference"
+
+
+def reference_root():
+    """The pglira/simpleICP checkout to build the reference from; None where its C++ sources are
+    absent or cannot be read (a directory the user may not enter is the same as none)."""
+    root = Path(os.environ.get("SIMPLEICP_REFERENCE") or DEFAULT_REFERENCE)
+    try:
+        return root if (root / "c++" / "src" / "simpleicp.cpp").is_file() else None
+    except OSError:
+        return None
+
+
+REF = reference_root()
 GOLD = REPO / "tests" / "golden"
 OUT = REPO / "oracle" / "_ref"
 sys.path.insert(0, str(REPO / "tests"))
@@ -118,13 +134,16 @@ def pack(j, cli_screen, api_screen, params):
         converged=np.bool_(j["converged"]),
         cli_screen=np.str_(cli_screen),
         params_repr=np.str_(repr(params)),
-        recipe=np.str_("oracle/make_golden_cpp.py: unmodified /root/reference/c++/src compiled by "
+        recipe=np.str_("oracle/make_golden_cpp.py: unmodified c++/src of pglira/simpleICP compiled by "
                        "oracle/Makefile against oracle/cpp_standin"),
     )
 
 
 def main(names):
     from conftest import load_pair  # the committed lossless input fixtures (== the .xyz files)
+
+    if REF is None:
+        sys.exit(f"no readable pglira/simpleICP checkout at {DEFAULT_REFERENCE}: set SIMPLEICP_REFERENCE")
 
     cli, driver = build()
     for name in names:

@@ -28,7 +28,7 @@ SYMBOLS = (
     "sicp_set_normals", "sicp_set_mov_normals", "sicp_get_knn", "sicp_match", "sicp_reject", "sicp_solve",
     "sicp_uncertainties", "sicp_run", "sicp_get_transform", "sicp_get_residuals", "sicp_iterate", "sicp_transform",
     "sicp_select_n_points", "sicp_register",
-    "sicp_register_batch", "sicp_get_timings", "sicp_time_stages", "sicp_get_phase_times",
+    "sicp_register_batch", "sicp_get_timings", "sicp_time_stages", "sicp_get_iteration", "sicp_get_phase_times",
     "sicp_xyz_load", "sicp_xyz_free", "sicp_xyz_save", "sicp_io_last_error",
 )
 
@@ -149,6 +149,7 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
                                 C.POINTER(RegisterParams), C.POINTER(PairResult)],
         "sicp_get_timings": [vp, C.POINTER(Timings)],
         "sicp_time_stages": [vp, C.POINTER(RunParams), i32, i32, C.POINTER(dbl)],
+        "sicp_get_iteration": [vp, C.POINTER(IterRecord), C.POINTER(dbl), vp, vp, vp],
         "sicp_get_phase_times": [vp, C.POINTER(dbl)],
     }
     for name, args in sigs.items():
@@ -507,6 +508,18 @@ class Engine:
         self._check(self._lib.sicp_time_stages(self._h, C.byref(params), int(reps),
                                                (1 if flush_l2 else 0) | (2 if outer_only else 0), ms))
         return {"match_grid": ms[0], "bruteforce_pass": ms[1], "reject_solve": ms[2], "iteration": ms[3]}
+
+    def last_iteration(self):
+        """What the last iterate / time_stages iteration computed, read back without running
+        anything: (record, 4 x 4 cumulative transform, matched movable index, point-to-plane
+        distance, keep flag), the arrays with one entry per selected point."""
+        rec = IterRecord()
+        T = (C.c_double * 16)()
+        idx = np.empty(self.K, dtype=np.int64)
+        d = np.empty(self.K, dtype=np.float64)
+        keep = np.empty(self.K, dtype=np.uint8)
+        self._check(self._lib.sicp_get_iteration(self._h, C.byref(rec), T, _ptr(idx), _ptr(d), _ptr(keep)))
+        return rec, np.array(T).reshape(4, 4), idx, d, keep.astype(bool)
 
     def phase_times(self) -> list:
         """Diagnostics: block-0 phase stamps (us) of the last reject+solve kernel."""

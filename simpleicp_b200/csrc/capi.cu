@@ -124,6 +124,7 @@ void wait_background_upload(Ctx& c) {
 
 void init_state(Ctx& c, const double x[6], const Rigid* T_or_null, bool reset_loop) {
   c.unresolved_clean = false;
+  c.stepped = false;
   // small pageable H2D copies are staged by the runtime before the call returns
   DevState h;
   if (reset_loop) {
@@ -399,7 +400,7 @@ int32_t sicp_set_selected(sicp_ctx* ctx, const int64_t* idx, int64_t K) {
   gather_queries_launch(c);
   c.have_normals = false;
   c.nn_pos_valid = false;
-  c.matched = c.rejected = c.solved = false;
+  c.matched = c.rejected = c.solved = c.stepped = false;
   sync(c);
   API_END
 }
@@ -437,7 +438,7 @@ int32_t sicp_set_clouds(sicp_ctx* ctx, const double* fix_xyz, int64_t n_fix, con
   c.have_normals = false;
   c.mov_attr = false;
   c.nn_pos_valid = false;
-  c.matched = c.rejected = c.solved = false;
+  c.matched = c.rejected = c.solved = c.stepped = false;
   API_END
 }
 
@@ -518,7 +519,7 @@ int32_t sicp_set_mov_normals(sicp_ctx* ctx, const float* nx, const float* ny, co
   if (!nx && !ny && !nz && !planarity) {  // back to the default run
     c.mov_attr = false;
     c.mov_cos_max = -1.0;
-    c.matched = c.rejected = c.solved = false;
+    c.matched = c.rejected = c.solved = c.stepped = false;
     return SICP_OK;
   }
   SICP_REQUIRE(nx && ny && nz && planarity, SICP_ERR_BAD_ARG, "NULL normal array");
@@ -535,7 +536,7 @@ int32_t sicp_set_mov_normals(sicp_ctx* ctx, const float* nx, const float* ny, co
   SICP_CUDA(cudaGetLastError());
   c.mov_attr = true;
   c.mov_cos_max = (max_angle_rad >= 0.0) ? (max_angle_rad >= 1.5707963267948966 ? 0.0 : cos(max_angle_rad)) : -1.0;
-  c.matched = c.rejected = c.solved = false;
+  c.matched = c.rejected = c.solved = c.stepped = false;
   sync(c);
   API_END
 }
@@ -590,6 +591,7 @@ int32_t sicp_reject(sicp_ctx* ctx, double min_planarity, uint8_t* keep, int64_t*
   }
   c.min_planarity_last = min_planarity;
   c.rejected = true;
+  c.stepped = false;
   API_END
 }
 
@@ -642,6 +644,7 @@ int32_t sicp_solve(sicp_ctx* ctx, const sicp_lsq_params* lp, double x[6], double
     sync(c);
   }
   c.solved = true;
+  c.stepped = false;
   API_END
 }
 
@@ -664,7 +667,7 @@ int32_t sicp_iterate(sicp_ctx* ctx, const sicp_run_params* p, const double x_in[
   }
   if (x_in) c.expect_unresolved = true;
   launch_iteration(c, *p, ctx->it_counter, false, 0, true, false);
-  c.matched = c.rejected = true;
+  c.matched = c.rejected = c.stepped = true;
   if (rec) {
     DevState h;
     fetch_records(c, 0, 1);
@@ -810,6 +813,7 @@ static void run_loop(sicp_ctx* ctx, Ctx& c, const sicp_run_params* p, sicp_run_r
   c.tm.reject_solve_ms = ms;
   if (log) std::memcpy(log, c.rec_host, sizeof(sicp_iter_record) * done);
   c.matched = c.rejected = c.solved = true;
+  c.stepped = false;
 }
 
 int32_t sicp_run(sicp_ctx* ctx, const sicp_run_params* p, sicp_run_result* out,
@@ -876,7 +880,7 @@ int32_t sicp_select_n_points(sicp_ctx* ctx, int64_t n, int64_t* idx_out) {
     gather_queries_launch(c);
     c.have_normals = false;
     c.nn_pos_valid = false;
-    c.matched = c.rejected = c.solved = false;
+    c.matched = c.rejected = c.solved = c.stepped = false;
   }
   if (idx_out) copy_any(c, idx_out, c.sel_idx.p, sizeof(long long) * c.K);
   sync(c);
@@ -909,7 +913,7 @@ int32_t sicp_register(sicp_ctx* ctx, const double* fix_xyz, int64_t n_fix, const
   c.have_normals = false;
   c.mov_attr = false;
   c.nn_pos_valid = false;
-  c.matched = c.rejected = c.solved = false;
+  c.matched = c.rejected = c.solved = c.stepped = false;
   // Transfers in the order the pipeline consumes them.  The fixed cloud goes first on the
   // context's stream; the movable cloud follows on the copy stream, and while it crosses PCIe the
   // fixed-side work (subsample, k-NN + PCA normals) runs.  With the overlap filter the selection
@@ -1066,7 +1070,23 @@ int32_t sicp_time_stages(sicp_ctx* ctx, const sicp_run_params* p, int32_t reps, 
   }
   for (auto& ev : e) cudaEventDestroy(ev);
   for (int i = 0; i < 4; ++i) ms[i] = acc[i] / reps;
-  c.matched = c.rejected = true;
+  c.matched = c.rejected = c.stepped = true;
+  API_END
+}
+
+int32_t sicp_get_iteration(sicp_ctx* ctx, sicp_iter_record* rec, double T[16], int64_t* nn_idx,
+                           double* dist, uint8_t* keep) {
+  API_BEGIN(ctx)
+  SICP_REQUIRE(c.stepped, SICP_ERR_STATE, "no sicp_iterate / sicp_time_stages iteration to read back");
+  DevState h;
+  fetch_records(c, 0, 1);
+  SICP_CUDA(cudaMemcpyAsync(&h, c.dev_state.p, sizeof(h), cudaMemcpyDeviceToHost, c.stream));
+  if (nn_idx) copy_any(c, nn_idx, c.nn_idx.p, sizeof(long long) * c.K);
+  if (dist) copy_any(c, dist, c.dist.p, sizeof(double) * c.K);
+  if (keep) copy_any(c, keep, c.keep.p, (size_t)c.K);
+  sync(c);
+  if (rec) *rec = c.rec_host[0];
+  if (T) H_from_rigid(h.T, T);
   API_END
 }
 

@@ -114,6 +114,9 @@ struct Ctx {
   DevBuf<unsigned char> bf_scratch;
   long long n_kept = 0;
   bool matched = false, rejected = false, solved = false;
+  // record slot 0, dev_state and nn_idx / dist / keep are those of the last sicp_iterate or
+  // sicp_time_stages iteration (what sicp_get_iteration reads back)
+  bool stepped = false;
   bool expect_unresolved = true;  // last known: did some query exceed the ring limit?
   double min_planarity_last = 0.0;
 

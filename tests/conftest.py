@@ -8,7 +8,6 @@ import pytest
 REPO = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(REPO))
 GOLD = REPO / "tests" / "golden"
-REFERENCE = Path("/root/reference")
 
 TRAVEL = ("dragon", "bunny", "multisensor", "webots")
 ALIAS = {"dragon_observed": "dragon", "dragon_movnormals": "dragon"}

@@ -1,6 +1,6 @@
 """Pins oracle/linearized_oracle.py (the restatement of the linearised simpleICP variant) to the
 UNMODIFIED C++ reference: tests/golden/cppref_<name>.npz were written by
-oracle/make_golden_cpp.py from /root/reference/c++/src compiled by oracle/Makefile against the
+oracle/make_golden_cpp.py from the reference's c++/src compiled by oracle/Makefile against the
 stand-in dependency headers in oracle/cpp_standin (Eigen, nanoflann and cxxopts are not in the
 image).  Configurations: the four command lines of c++/run_simpleicp.sh:11-41 (dragon, airborne,
 terrestrial, bunny with --max_overlap_distance 1) plus two with non-default flags.
@@ -32,6 +32,7 @@ from conftest import load_pair
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT / "oracle"))
 import linearized_oracle as lo  # noqa: E402
+import make_golden_cpp as mg  # noqa: E402
 
 GOLD = ROOT / "tests" / "golden"
 DATA = {"dragon_k5000": "dragon", "bunny_maxit3": "bunny"}
@@ -144,14 +145,11 @@ def test_standalone_restatement_reaches_the_same_registration():
         assert np.abs(r.T - T).max() < tol
 
 
-@pytest.mark.skipif(not Path("/root/reference/c++/src/simpleicp.cpp").exists() or shutil.which("g++") is None,
-                    reason="needs the reference tree and g++ (build container only)")
+@pytest.mark.skipif(mg.REF is None or shutil.which("g++") is None,
+                    reason="needs g++ and a readable pglira/simpleICP checkout (oracle/make_golden_cpp.py)")
 def test_fixture_is_reproduced_by_the_recipe(tmp_path):
-    """Re-run the recipe: build oracle/_ref from the sources under /root/reference and compare the
+    """Re-run the recipe: build oracle/_ref from the reference's C++ sources and compare the
     dragon fixture field by field -- the committed numbers are the compiled reference's."""
-    sys.path.insert(0, str(ROOT / "oracle"))
-    import make_golden_cpp as mg
-
     cli, driver = mg.build()
     fix, mov, flags = mg.CONFIGS["dragon"]
     X_fix, X_mov = load_pair("dragon")
@@ -166,6 +164,6 @@ def test_fixture_is_reproduced_by_the_recipe(tmp_path):
     # the reference CLI's own error path (simpleicp.cpp:26-36 -> simpleicp-cli.cpp:60-64)
     far = tmp_path / "far.xyz"
     np.savetxt(far, X_mov[:2000] + 1e4, fmt="%.4f")
-    r = subprocess.run([str(cli), "--fixed", "/root/reference/data/dragon1.xyz", "--movable", str(far),
+    r = subprocess.run([str(cli), "--fixed", str(mg.REF / "data" / "dragon1.xyz"), "--movable", str(far),
                         "--max_overlap_distance", "1"], capture_output=True, text=True)
     assert r.returncode == 1 and "Point clouds do not overlap within max_overlap_distance" in r.stderr

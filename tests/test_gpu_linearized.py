@@ -89,7 +89,7 @@ CPPREF = {  # fixture -> input pair (oracle/make_golden_cpp.py: c++/run_simpleic
 @pytest.mark.parametrize("name", list(CPPREF))
 def test_against_the_compiled_cpp_reference(gpu, name):
     """The CUDA path against the per-iteration output of the unmodified C++ reference (compiled
-    from /root/reference/c++/src by oracle/Makefile, run by oracle/make_golden_cpp.py).  The
+    from the reference's c++/src by oracle/Makefile, run by oracle/make_golden_cpp.py).  The
     reference run's normals are handed over (rounded to the float32 the library stores): the
     eigenvector sign is implementation defined on both sides.  Measured on the CPU restatement,
     that rounding moves H by < 1e-9 on these inputs and no kept count at all, so: selection,
@@ -234,7 +234,7 @@ def test_reference_cpp_cli_linked_against_the_library(gpu, tmp_path):
     """INTEGRATION.md section 5 as a running program: the reference's own, unmodified CLI main()
     (c++/src/simpleicp-cli.cpp) linked with integration/cpp/simpleicp_b200_binding.cpp -- the
     reference's SimpleICP() signature implemented on the C ABI -- instead of its CPU sources
-    (oracle/Makefile -> oracle/_ref/simpleicp_cpp_b200, built where /root/reference exists).  Its
+    (oracle/Makefile -> oracle/_ref/simpleicp_cpp_b200, built where the reference checkout is readable).  Its
     screen output must be the library's linearised run, and agree with the CPU build of the same
     CLI (tests/golden/cppref_dragon.npz) as far as the eigenvector sign convention allows."""
     import re
@@ -244,7 +244,7 @@ def test_reference_cpp_cli_linked_against_the_library(gpu, tmp_path):
 
     exe = REPO / "oracle" / "_ref" / "simpleicp_cpp_b200"
     if not exe.exists():
-        pytest.skip("oracle/_ref/simpleicp_cpp_b200 not built (needs the reference tree at build time)")
+        pytest.skip("oracle/_ref/simpleicp_cpp_b200 not built (needs the reference checkout at build time)")
     X_fix, X_mov = load_pair("dragon")
     f1, f2 = tmp_path / "dragon1.xyz", tmp_path / "dragon2.xyz"
     sb.write_xyz(f1, X_fix, decimals=4, header=False)

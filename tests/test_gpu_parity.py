@@ -351,6 +351,41 @@ def test_predicted_histogram_select_is_used_and_exact(gpu):
             assert st[0] == np.median(d[S1]) and st[1] == np.median(np.abs(d[S1] - st[0]))
 
 
+def test_last_iteration_read_back(gpu):
+    """sicp_get_iteration hands back what the last iterate / time_stages iteration computed: the
+    record iterate returned, the transform of its parameters, and the match and keep mask the
+    stage API computes from the transform that iteration started from.  A call that changes the
+    loop state makes it an error."""
+    X_fix, X_mov = load_pair("dragon")
+    with _capi.Engine() as e:
+        e.set_clouds(X_fix, X_mov)
+        e.set_selected(sb.pointcloud.subsample_indices(len(X_fix), 1000).astype(np.int64))
+        e.estimate_normals(10)
+        p = e.run_params(0.3, 1.0, 100, e.lsq_params(np.zeros(6), np.zeros(6), np.zeros(6), 1.0))
+        with pytest.raises(_capi.SicpError, match="read back"):
+            e.last_iteration()
+        e.iterate(p, x_in=np.zeros(6), want_record=True)
+        x_before = np.array(e.iterate(p, want_record=True).x)
+        rec = e.iterate(p, want_record=True)
+        got, T, idx, d, keep = e.last_iteration()
+        for f in ("n_kept", "median", "mad", "mean_dist", "std_dist", "mean_res", "std_res"):
+            assert getattr(got, f) == getattr(rec, f), f
+        assert list(got.x) == list(rec.x)
+        np.testing.assert_allclose(T, O.rbp_to_H(np.array(rec.x)), rtol=0, atol=1e-12)
+        e.time_stages(p, 2, False, outer_only=True)
+        got2, T2, *_ = e.last_iteration()
+        np.testing.assert_allclose(T2, O.rbp_to_H(np.array(got2.x)), rtol=0, atol=1e-12)
+        # (the host rebuilds H with NumPy's sin/cos: distances agree to ~1e-16, ties may pick another index)
+        idx_m, d_m = e.match(O.rbp_to_H(x_before))
+        same = idx == idx_m
+        assert same.mean() > 0.99
+        np.testing.assert_allclose(d[same], d_m[same], rtol=0, atol=1e-12)
+        keep_m, n_kept, _ = e.reject(0.3)
+        assert np.array_equal(keep, keep_m) and n_kept == got.n_kept
+        with pytest.raises(_capi.SicpError, match="read back"):
+            e.last_iteration()
+
+
 def test_host_sync_batching_is_equivalent(gpu):
     """Queuing several iterations between host reads (device-side stop flag) changes nothing."""
     g = load_golden("dragon")
