@@ -251,20 +251,24 @@ int32_t sicp_register(sicp_ctx* ctx, const double* fix_xyz /*[h|d] n_fix x 3*/, 
                       int64_t* n_selected /*[h] or NULL*/);
 
 /* ---- many independent pairs in one call (BASELINE.json configs[4]; SURVEY.md section 8e) --------
- * SimpleICP.run (simpleicp.py:75-324, defaults: no overlap filter) for n_pairs independent
- * (fixed, movable) pairs on ONE GPU with ONE set of kernel launches per stage and per iteration
- * for the whole batch: the grids of all 2 n_pairs clouds are built in one segmented counting
- * sort, the searches of all pairs run in one launch, reject + solve run one block per pair, every
- * pair has its own stop flag.  Results per pair equal those of sicp_register on that pair.
+ * SimpleICP.run (simpleicp.py:75-324) for n_pairs independent (fixed, movable) pairs on ONE GPU
+ * with ONE set of kernel launches per stage and per iteration for the whole batch: the grids of
+ * all 2 n_pairs clouds are built in one segmented counting sort, the searches of all pairs run in
+ * one launch, reject + solve run one block per pair, every pair has its own stop flag.  Results
+ * per pair equal those of sicp_register on that pair.
  * fix_xyz[i] / mov_xyz[i] point to the i-th pair's clouds (host, ideally pinned, or device);
- * correspondences must be <= 4096 (one block per pair) and max_overlap_distance must be unused.
- * out[i].status is the sicp_status of pair i (a pair without enough correspondences fails alone);
- * the call itself fails only on bad arguments or CUDA errors.                                   */
+ * correspondences must be <= 4096 (one block per pair).  A finite max_overlap_distance > 0 runs
+ * the partial-overlap filter of sicp_register on every pair (simpleicp.py:150-170, from the
+ * initial transform of p->run.lsq.x0, one distance and one initial transform for the whole call).
+ * out[i].status is the sicp_status of pair i (a pair without enough correspondences, or whose
+ * clouds do not overlap within max_overlap_distance, fails alone); the call itself fails only on
+ * bad arguments or CUDA errors.                                                                   */
 typedef struct {
   int32_t status;
   int32_t iterations;
   int32_t converged;
-  int32_t reserved;
+  int32_t n_selected;         /* fixed points the loop used (sicp_register's n_selected); 0 when
+                                 status is SICP_ERR_NO_OVERLAP                                     */
   int64_t n_kept;
   double H[16];
   double x[6];

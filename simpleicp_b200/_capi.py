@@ -71,7 +71,7 @@ class Timings(C.Structure):
 
 class PairResult(C.Structure):
     _fields_ = [("status", C.c_int32), ("iterations", C.c_int32), ("converged", C.c_int32),
-                ("reserved", C.c_int32), ("n_kept", C.c_int64), ("H", C.c_double * 16),
+                ("n_selected", C.c_int32), ("n_kept", C.c_int64), ("H", C.c_double * 16),
                 ("x", C.c_double * 6), ("sigma", C.c_double * 6), ("mean_res", C.c_double),
                 ("std_res", C.c_double)]
 
@@ -461,11 +461,12 @@ class Engine:
         self._check(self._lib.sicp_get_residuals(self._h, _ptr(res), res.size, C.byref(n)))
         return out, [log[i] for i in range(out.iterations)], res, transform_out
 
-    def register_batch(self, pairs, correspondences, neighbors, params: RunParams):
+    def register_batch(self, pairs, correspondences, neighbors, params: RunParams, max_overlap_distance=-1.0):
         """sicp_register_batch: SimpleICP.run for every (X_fix, X_mov) of `pairs` with one set of
         kernel launches per stage for the whole batch.  Clouds are NumPy arrays (pinned ones
-        upload at link speed) or CUDA tensors; nothing is copied on the host.  Returns the
-        ctypes array of PairResult (status per pair)."""
+        upload at link speed) or CUDA tensors; nothing is copied on the host.  A finite
+        `max_overlap_distance` > 0 filters every pair's fixed points as sicp_register does.
+        Returns the ctypes array of PairResult (status per pair)."""
         n = len(pairs)
         keep = [(_as_f64_xyz(a), _as_f64_xyz(b)) for a, b in pairs]  # keeps converted copies alive
         fp = (C.c_void_p * n)(*[_ptr(a) for a, _ in keep])
@@ -475,7 +476,7 @@ class Engine:
         rp = RegisterParams()
         rp.correspondences = int(correspondences)
         rp.neighbors = int(neighbors)
-        rp.max_overlap_distance = -1.0
+        rp.max_overlap_distance = float(max_overlap_distance)
         rp.run = params
         out = (PairResult * n)()
         self._check(self._lib.sicp_register_batch(self._h, n, fp, nf, mp, nm, C.byref(rp), out))

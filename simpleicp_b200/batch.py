@@ -125,9 +125,10 @@ def simpleicp_batch(
 
     `engine="batched"` (default) hands the rank's share to the library's batched engine in chunks
     of `batch_size` pairs (sicp_register_batch: one set of kernel launches per stage and per
-    iteration for the whole chunk, a block per pair for reject + solve, per-pair stop flags);
-    pairs it does not cover (overlap filter, more than 4096 correspondences, debug output) and
-    `engine="pool"` use the concurrent per-pair engines described above.
+    iteration for the whole chunk, a block per pair for reject + solve, per-pair stop flags),
+    with or without the overlap filter (`max_overlap_distance`); pairs it does not cover (more
+    than 4096 correspondences, debug output) and `engine="pool"` use the concurrent per-pair
+    engines described above.
 
     A pair that cannot be registered (no overlap, fewer than 6 correspondences: ordinary
     data-dependent outcomes) gets a NaN record whose `iterations` field is minus the library's
@@ -218,10 +219,8 @@ _BATCH_KEYS = {"correspondences", "neighbors", "min_planarity", "min_change", "m
 
 def _batchable(kw) -> bool:
     """Can the batched engine serve these run() arguments?  (One block per pair: at most 4096
-    correspondences; no overlap filter; nothing that needs per-pair host interaction.)"""
+    correspondences; nothing that needs per-pair host interaction.)"""
     if set(kw) - _BATCH_KEYS:
-        return False
-    if np.isfinite(kw.get("max_overlap_distance", np.inf)):
         return False
     return int(kw.get("correspondences", 1000)) <= 4096 and not kw.get("want_normals", False)
 
@@ -250,7 +249,8 @@ def _run_batched(get, mine, local, device, batch_size, kw, messages):
         for lo in range(0, len(mine), max(1, int(batch_size))):
             ids = range(lo, min(lo + max(1, int(batch_size)), len(mine)))
             pairs = [get(mine[j]) for j in ids]
-            res = eng.register_batch(pairs, kw.get("correspondences", 1000), kw.get("neighbors", 10), params)
+            res = eng.register_batch(pairs, kw.get("correspondences", 1000), kw.get("neighbors", 10), params,
+                                     float(kw.get("max_overlap_distance", np.inf)))
             for j, r in zip(ids, res):
                 if r.status == 0:
                     local[j] = pack_record(np.array(r.H).reshape(4, 4), r.iterations, r.n_kept, r.mean_res, r.std_res)

@@ -9,6 +9,8 @@
 //   upload        one cudaMemcpyAsync per cloud straight from the caller's (pinned) arrays; the
 //                 movable clouds cross PCIe while the fixed-side work runs
 //   grids         segmented counting sort over all clouds of a side (grid.cu: grid_build_batch)
+//   overlap       (max_overlap_distance only) keep flags of all fixed points in one launch, one
+//                 scan over the batch, ordered kept lists; per-pair K set on the device (nn.cu)
 //   select+gather rint(linspace) picks and their coordinates, all pairs in one launch
 //   normals       k-NN + PCA, blockIdx.y = pair
 //   loop          per iteration ONE match launch over (pair, query) and ONE reject/solve launch
@@ -52,8 +54,8 @@ static void register_batch(Ctx& c, int n_pairs, const double* const* fix_xyz, co
   SICP_REQUIRE(fix_xyz && n_fix && mov_xyz && n_mov && rp && out, SICP_ERR_BAD_ARG, "NULL argument");
   SICP_REQUIRE(rp->correspondences >= 1 && rp->correspondences <= 4096, SICP_ERR_BAD_ARG,
                "the batched engine runs one block per pair: correspondences must be in [1, 4096]");
-  SICP_REQUIRE(!(rp->max_overlap_distance > 0 && std::isfinite(rp->max_overlap_distance)), SICP_ERR_BAD_ARG,
-               "the batched engine has no overlap filter: register such pairs one by one");
+  // the same rule as sicp_register: anything else means the clouds fully overlap
+  const bool overlap = rp->max_overlap_distance > 0 && std::isfinite(rp->max_overlap_distance);
   const sicp_run_params& p = rp->run;
   SICP_REQUIRE(p.max_iterations >= 1 && p.max_iterations <= 4096, SICP_ERR_BAD_ARG,
                "max_iterations must be in [1, 4096]");
@@ -136,10 +138,16 @@ static void register_batch(Ctx& c, int n_pairs, const double* const* fix_xyz, co
     h.H_rep = h.T;
     std::vector<DevState> hs((size_t)n_pairs, h);
     SICP_CUDA(cudaMemcpyAsync(b.state.p, hs.data(), sizeof(DevState) * (size_t)n_pairs, cudaMemcpyHostToDevice, st));
+    if (overlap) {
+      b.fix_off.reserve((size_t)n_pairs + 1);
+      SICP_CUDA(cudaMemcpyAsync(b.fix_off.p, fo.data(), sizeof(long long) * ((size_t)n_pairs + 1), cudaMemcpyHostToDevice, st));
+    }
     SICP_CUDA(cudaStreamSynchronize(st));  // hs is a local (also: the fixed clouds have arrived)
   }
 
-  // ---- fixed side: grids, subsample + gather, normals (the movable clouds are still in flight)
+  // ---- fixed side: grids, subsample + gather, normals (the movable clouds are still in flight).
+  // With the overlap filter the selection needs the movable grids: fixed grids, movable grids,
+  // filter, select + gather, normals.
   std::vector<PairDev> pd((size_t)n_pairs);
   std::vector<BatchHostCloud> clouds((size_t)n_pairs);
   std::vector<GridView> views;
@@ -160,13 +168,17 @@ static void register_batch(Ctx& c, int n_pairs, const double* const* fix_xyz, co
     d.mov_off = mo[(size_t)i];
     d.K = std::min<long long>(rp->correspondences, n_fix[i]);
     d.q_off = (long long)i * Kmax;
+    d.n_cand = n_fix[i];
   }
-  SICP_CUDA(cudaMemcpyAsync(b.pairs.p, pd.data(), sizeof(PairDev) * (size_t)n_pairs, cudaMemcpyHostToDevice, st));
-  batch_select_gather_launch(c, b, rp->correspondences, c.variant != SICP_VARIANT_PYTHON);
-  {
+  auto fixed_side = [&]() {
+    batch_select_gather_launch(c, b, rp->correspondences, c.variant != SICP_VARIANT_PYTHON, overlap);
     StageTimer t(c, &c.tm.normals_ms);
     batch_normals_launch(c, b, rp->neighbors);
     t.stop();
+  };
+  if (!overlap) {
+    SICP_CUDA(cudaMemcpyAsync(b.pairs.p, pd.data(), sizeof(PairDev) * (size_t)n_pairs, cudaMemcpyHostToDevice, st));
+    fixed_side();
   }
 
   // ---- movable side
@@ -182,6 +194,15 @@ static void register_batch(Ctx& c, int n_pairs, const double* const* fix_xyz, co
     for (int a = 0; a < 3; ++a) pd[(size_t)i].cm[a] = centres[(size_t)i * 3 + a];
   }
   SICP_CUDA(cudaMemcpyAsync(b.pairs.p, pd.data(), sizeof(PairDev) * (size_t)n_pairs, cudaMemcpyHostToDevice, st));
+  c.tm.overlap_ms = 0;
+  if (overlap) {
+    // the filter sets K, n_cand and kept_off of every descriptor on the device: nothing re-uploads
+    // them after this point
+    StageTimer t(c, &c.tm.overlap_ms);
+    batch_overlap_launch(c, b, rp->correspondences, rp->max_overlap_distance);
+    t.stop();
+    fixed_side();
+  }
 
   // ---- the loop: two launches per iteration for the whole batch
   cudaEvent_t e0, e1;

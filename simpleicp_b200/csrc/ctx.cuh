@@ -173,9 +173,11 @@ struct PairDev {
   GridView gmov, gfix;
   long long n_fix, n_mov;
   long long fix_off, mov_off;  // first point of this pair in the concatenated clouds
-  long long K;                 // selected fixed points (<= Kmax)
+  long long K;                 // selected fixed points (<= Kmax); 0: no fixed point within max_overlap_distance
   long long q_off;             // first entry of this pair in the per-query arrays
   double cm[3];                // centre of the movable grid's box (moment centring)
+  long long n_cand;            // fixed points the selection thins: n_fix, or the overlap filter's kept count
+  long long kept_off;          // overlap filter: first entry of this pair's kept list (Batch::ov_kept)
 };
 
 // One cloud of a batched grid build (filled by the host from the bounding boxes).
@@ -212,6 +214,14 @@ struct Batch {
   int bin_cap = 0;
   DevBuf<uint32_t> nn_pos;
   DevBuf<uint8_t> keep;
+  // overlap filter, one entry per fixed point of the batch (total_fix)
+  DevBuf<long long> fix_off;      // n_pairs + 1: first fixed point of every pair, then total_fix
+  DevBuf<long long> ov_nn;        // nearest movable point (or the point that decided the bound)
+  DevBuf<double> ov_d2;           // its squared distance
+  DevBuf<uint32_t> ov_flag;       // 1: closer than max_overlap_distance
+  DevBuf<uint32_t> ov_scan;       // exclusive scan of ov_flag (total_fix + 1 entries)
+  DevBuf<uint32_t> ov_kept;       // global positions of the kept points, ascending
+  DevBuf<uint32_t> ov_block_sums;
   // per-pair state
   DevBuf<DevState> state;
   DevBuf<unsigned int> lin_hist;       // n_pairs x (LH_BINS + 2)
@@ -283,7 +293,14 @@ struct BatchHostCloud {
 };
 void grid_build_batch(Ctx& c, Batch& b, BatchGrid& bg, const std::vector<BatchHostCloud>& clouds,
                       std::vector<GridView>& views, std::vector<double>& centres /* 3 per cloud */);
-void batch_select_gather_launch(Ctx& c, Batch& b, long long correspondences, int round_away);
+void batch_select_gather_launch(Ctx& c, Batch& b, long long correspondences, int round_away, bool overlap);
+// PointCloud.select_in_range for every pair (needs both grids and the pairs' initial DevState):
+// keep flags for all fixed points in one launch, one scan over the batch, the ordered kept lists;
+// sets every pair's n_cand, kept_off and K = min(correspondences, kept count) on the device, and
+// stop = 2 for a pair that keeps nothing (reported as SICP_ERR_NO_OVERLAP).
+void batch_overlap_launch(Ctx& c, Batch& b, long long correspondences, double max_dist);
+// exclusive scan of n uint32 into out[0 .. n] (out[n] = the total); grid.cu
+void scan_u32(Ctx& c, const uint32_t* in, long long n, DevBuf<uint32_t>& block_sums, uint32_t* out);
 void batch_normals_launch(Ctx& c, Batch& b, int k);
 void batch_match_launch(Ctx& c, Batch& b, bool warm);
 void batch_rs_launch(Ctx& c, Batch& b, const sicp_run_params& p, int it, bool want_sigma);

@@ -468,6 +468,22 @@ inline double host_key_to_f64(unsigned long long k) {
 
 }  // namespace
 
+// The three-kernel scan plus the total: the batched grid build's cell table and the overlap
+// filter's kept lists (nn.cu: batch_overlap_launch) both come out of one scan over a whole batch.
+void scan_u32(Ctx& c, const uint32_t* in, long long n, DevBuf<uint32_t>& block_sums, uint32_t* out) {
+  cudaStream_t st = c.stream;
+  const long long nsb = (n + kScanItems - 1) / kScanItems;
+  block_sums.reserve(nsb + 1);
+  c.misc_counters.reserve(64);
+  SICP_CUDA(cudaMemsetAsync(c.misc_counters.p + 16, 0, sizeof(unsigned int), st));  // the kernel's (unused here) nonzero counter
+  k_scan_reduce<<<(unsigned)nsb, 256, 0, st>>>(in, n, block_sums.p, c.misc_counters.p + 16);
+  k_scan_blocksums<<<1, 1024, 0, st>>>(block_sums.p, (int)nsb);
+  k_scan_down<<<(unsigned)nsb, 256, 0, st>>>(in, n, block_sums.p, out);
+  k_scan_total<<<1, 32, 0, st>>>(in, n, out);
+  SICP_CUDA(cudaGetLastError());
+  c.tm.kernel_launches += 4;
+}
+
 void grid_build_batch(Ctx& c, Batch& b, BatchGrid& bg, const std::vector<BatchHostCloud>& clouds,
                       std::vector<GridView>& views, std::vector<double>& centres) {
   cudaStream_t st = c.stream;
@@ -577,18 +593,11 @@ void grid_build_batch(Ctx& c, Batch& b, BatchGrid& bg, const std::vector<BatchHo
     if (!again) break;
   }
   // exclusive scan of the concatenated counters -> global record positions
-  const long long nsb = (total_cells + kScanItems - 1) / kScanItems;
-  bg.block_sums.reserve(nsb + 1);
-  c.misc_counters.reserve(64);
-  SICP_CUDA(cudaMemsetAsync(c.misc_counters.p + 16, 0, sizeof(unsigned int), st));  // the kernel's (unused here) occupancy counter
-  k_scan_reduce<<<(unsigned)nsb, 256, 0, st>>>(bg.fill.p, total_cells, bg.block_sums.p, c.misc_counters.p + 16);
-  k_scan_blocksums<<<1, 1024, 0, st>>>(bg.block_sums.p, (int)nsb);
-  k_scan_down<<<(unsigned)nsb, 256, 0, st>>>(bg.fill.p, total_cells, bg.block_sums.p, bg.cell_table.p);
-  k_scan_total<<<1, 32, 0, st>>>(bg.fill.p, total_cells, bg.cell_table.p);
+  scan_u32(c, bg.fill.p, total_cells, bg.block_sums, bg.cell_table.p);
   SICP_CUDA(cudaMemsetAsync(bg.fill.p, 0, (size_t)total_cells * sizeof(uint32_t), st));
   k_scatter_batch<<<dim3((unsigned)((max_n + 255) / 256), nc), 256, 0, st>>>(b.plans.p, bg.cid.p, bg.cell_table.p, bg.fill.p, bg.recs.p);
   SICP_CUDA(cudaGetLastError());
-  c.tm.kernel_launches += 5;
+  c.tm.kernel_launches += 1;
   views.resize((size_t)nc);
   centres.resize((size_t)nc * 3);
   for (int i = 0; i < nc; ++i) {

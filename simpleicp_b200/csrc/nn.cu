@@ -586,6 +586,67 @@ __global__ void __launch_bounds__(128) k_match_batch(BatchMatchArgs a) {
                       co, gt);
 }
 
+// Overlap filter of a batch (PointCloud.select_in_range, pointcloud.py:149-171): every fixed point
+// of every pair is a query, read in place from the concatenated clouds.  The grid is flat over the
+// batch's fixed points (pairs are ragged: a grid sized by the largest pair would idle most blocks);
+// a query group finds its pair by bisection of the offsets.  The search only decides on which side
+// of cap2 = max_overlap_distance^2 the nearest distance lies (grid_nn); without a brute-force
+// hand-over a query far outside the movable box still ends once every unexplored cell lies beyond
+// the bound, after about max_overlap_distance / h rings.
+struct BatchOverlapArgs {
+  const PairDev* pairs;
+  const long long* fix_off;  // n_pairs + 1
+  int n_pairs;
+  const DevState* state;
+  const double* fix_xyz;
+  long long total;
+  long long* nn;
+  double* d2;
+  uint32_t* flag;
+  double cap2;
+};
+template <int MG>
+__global__ void __launch_bounds__(128) k_overlap_batch(BatchOverlapArgs a) {
+  const long long gt = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  const long long g = gt / MG;
+  if (g >= a.total) return;  // a whole group leaves together
+  int lo = 0, hi = a.n_pairs - 1;  // the last pair that starts at or before g
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (a.fix_off[mid] <= g) lo = mid;
+    else hi = mid - 1;
+  }
+  const long long f = a.fix_off[lo];
+  const GridView gv = a.pairs[lo].gmov;
+  const CorrOut co{nullptr, 0, nullptr, nullptr, 0, 0, nullptr, nullptr, -1.0};
+  match_coop_body<MG>(gv, a.state + lo, a.fix_xyz + 3 * f, nullptr, nullptr, a.fix_off[lo + 1] - f, 1 << 30, 0,
+                      a.nn + f, a.d2 + f, nullptr, nullptr, a.cap2, co, (g - f) * MG + (gt & (MG - 1)));
+  // lane 0 of the group stored the distance above
+  if ((threadIdx.x & (MG - 1)) == 0) a.flag[g] = (a.d2[g] < a.cap2) ? 1u : 0u;  // strict, as cKDTree's bound
+}
+
+// kept list: position scan[g] of the batch-wide list holds g
+__global__ void __launch_bounds__(256)
+    k_overlap_compact(const uint32_t* __restrict__ flag, const uint32_t* __restrict__ scan, long long total,
+                      uint32_t* __restrict__ kept) {
+  const long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (g < total && flag[g]) kept[scan[g]] = (uint32_t)g;
+}
+
+// per pair: m = kept count, its list starts at scan[fix_off]; K = min(correspondences, m).  A pair
+// that keeps nothing gets K = 0 and a raised stop flag, so every later kernel leaves it alone.
+__global__ void k_overlap_pairs(PairDev* __restrict__ pairs, DevState* __restrict__ state,
+                                const long long* __restrict__ fix_off, const uint32_t* __restrict__ scan,
+                                int n_pairs, long long correspondences) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_pairs) return;
+  const long long s0 = scan[fix_off[i]], m = (long long)scan[fix_off[i + 1]] - s0;
+  pairs[i].n_cand = m;
+  pairs[i].kept_off = s0;
+  pairs[i].K = min(correspondences, m);
+  if (m == 0) state[i].stop = 2;
+}
+
 // ------------------------------------------------------------------------------------------
 // brute-force engine (TMA staged)
 // ------------------------------------------------------------------------------------------
@@ -904,20 +965,23 @@ static void bf_launch(Ctx& c, bool with_distance, double* out, bool whole_set) {
 
 namespace {
 // per pair: sel[i] = rint(linspace(0, n_fix - 1, K)) (PointCloud.select_n_points, k_select_n in
-// capi.cu) and the gather of the selected fixed points, in one launch for the whole batch
+// capi.cu) and the gather of the selected fixed points, in one launch for the whole batch.  With
+// the overlap filter (kept != null) the linspace runs over the pair's kept list instead:
+// sel[i] = kept[rint(linspace(0, m - 1, K))[i]], m = the pair's kept count.
 __global__ void __launch_bounds__(256)
     k_select_gather_batch(const PairDev* __restrict__ pairs, const double* __restrict__ fix_xyz, int away,
-                          long long* __restrict__ sel, double* __restrict__ q_xyz) {
+                          const uint32_t* __restrict__ kept, long long* __restrict__ sel, double* __restrict__ q_xyz) {
   const PairDev pd = pairs[blockIdx.y];
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i >= pd.K) return;
-  const long long m = pd.n_fix, n = pd.K;
+  const long long m = pd.n_cand, n = pd.K;
   long long j = i;
   if (n < m) {
     const double step = (n > 1) ? (double)(m - 1) / (double)(n - 1) : 0.0;
     const double y = (i == n - 1 && n > 1) ? (double)(m - 1) : (double)i * step;
     j = (long long)(away ? round(y) : rint(y));
   }
+  if (kept) j = (long long)kept[pd.kept_off + j] - pd.fix_off;
   sel[pd.q_off + i] = j;
   const double* __restrict__ src = fix_xyz + 3 * (pd.fix_off + j);
   double* __restrict__ dst = q_xyz + 3 * (pd.q_off + i);
@@ -927,12 +991,45 @@ __global__ void __launch_bounds__(256)
 }
 }  // namespace
 
-void batch_select_gather_launch(Ctx& c, Batch& b, long long correspondences, int round_away) {
+void batch_select_gather_launch(Ctx& c, Batch& b, long long correspondences, int round_away, bool overlap) {
   (void)correspondences;
   k_select_gather_batch<<<dim3((unsigned)((b.Kmax + 255) / 256), b.n_pairs), 256, 0, c.stream>>>(
-      b.pairs.p, b.fix_xyz.p, round_away, b.sel_idx.p, b.q_xyz.p);
+      b.pairs.p, b.fix_xyz.p, round_away, overlap ? b.ov_kept.p : nullptr, b.sel_idx.p, b.q_xyz.p);
   SICP_CUDA(cudaGetLastError());
   c.tm.kernel_launches += 1;
+}
+
+void batch_overlap_launch(Ctx& c, Batch& b, long long correspondences, double max_dist) {
+  const long long total = b.total_fix;
+  b.ov_nn.reserve(total);
+  b.ov_d2.reserve(total);
+  b.ov_flag.reserve(total);
+  b.ov_scan.reserve(total + 1);
+  b.ov_kept.reserve(total);
+  BatchOverlapArgs a;
+  a.pairs = b.pairs.p;
+  a.fix_off = b.fix_off.p;
+  a.n_pairs = b.n_pairs;
+  a.state = b.state.p;
+  a.fix_xyz = b.fix_xyz.p;
+  a.total = total;
+  a.nn = b.ov_nn.p;
+  a.d2 = b.ov_d2.p;
+  a.flag = b.ov_flag.p;
+  a.cap2 = max_dist * max_dist;
+  // lanes per query: 16 while few queries are in flight, else 8 (with 4 or 2 lanes the search body
+  // spills a few registers in this kernel)
+  const int mg = (total <= 16384) ? 16 : 8;
+  const unsigned blocks = (unsigned)((total * mg + 127) / 128);
+  if (mg == 8) k_overlap_batch<8><<<blocks, 128, 0, c.stream>>>(a);
+  else k_overlap_batch<16><<<blocks, 128, 0, c.stream>>>(a);
+  SICP_CUDA(cudaGetLastError());
+  scan_u32(c, b.ov_flag.p, total, b.ov_block_sums, b.ov_scan.p);
+  k_overlap_compact<<<(unsigned)((total + 255) / 256), 256, 0, c.stream>>>(b.ov_flag.p, b.ov_scan.p, total, b.ov_kept.p);
+  k_overlap_pairs<<<(b.n_pairs + 127) / 128, 128, 0, c.stream>>>(b.pairs.p, b.state.p, b.fix_off.p, b.ov_scan.p,
+                                                                  b.n_pairs, correspondences);
+  SICP_CUDA(cudaGetLastError());
+  c.tm.kernel_launches += 3;
 }
 
 void batch_match_launch(Ctx& c, Batch& b, bool warm) {

@@ -2032,11 +2032,12 @@ __global__ void __launch_bounds__(256)
     sicp_pair_result r;
     r.iterations = st.iterations_done;
     r.converged = (st.stop == 1) ? 1 : 0;
-    r.reserved = 0;
+    r.n_selected = (int32_t)K;
     r.n_kept = st.n_kept;
     // fewer than 6 correspondences at some iteration (stop 2, or an iteration that never finished)
     const bool too_few = (st.stop == 2) || (!st.stop && st.iterations_done < max_iterations) || !have;
     r.status = too_few ? SICP_ERR_TOO_FEW_CORR : (st.lm_ok ? SICP_OK : SICP_ERR_SINGULAR);
+    if (K == 0) r.status = SICP_ERR_NO_OVERLAP;  // the overlap filter kept no fixed point: the pair never ran
     const Rigid& H = variant ? st.H_rep : st.T;
     for (int a = 0; a < 3; ++a) {
       for (int c2 = 0; c2 < 3; ++c2) r.H[a * 4 + c2] = H.r[a * 3 + c2];

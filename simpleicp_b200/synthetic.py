@@ -9,11 +9,12 @@ import numpy as np
 from . import mathutils
 
 
-def surface(n: int, seed: int, extent: float = 100.0) -> np.ndarray:
+def surface(n: int, seed: int, extent: float = 100.0, x0: float = 0.0) -> np.ndarray:
     """Tilted, gently undulating plane with 1 cm noise (all six rigid-body parameters are
-    observable on it; a perfect plane would leave three of them free)."""
+    observable on it; a perfect plane would leave three of them free), sampled over
+    [x0, x0 + extent] x [0, extent]: patches with different x0 overlap partly."""
     rng = np.random.default_rng(seed)
-    x = rng.uniform(0, extent, n)
+    x = rng.uniform(x0, x0 + extent, n)
     y = rng.uniform(0, extent, n)
     z = 0.05 * x + 0.03 * y + 2 * np.sin(2 * np.pi * x / 25) * np.cos(2 * np.pi * y / 40)
     z = z + rng.normal(0, 0.01, n)
